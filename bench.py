@@ -1,11 +1,18 @@
 """bench.py - LLaMA-7B gptq.int4 batch-1 decode throughput on B200 (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one decoded token (one pass of generate()'s loop body, generate.py:63-89: model forward + top-k / softmax /
-multinomial sampling) on random-init 7B gptq.int4 weights, KV cache S = 2048.  The K timed steps are spread EVENLY over
+multinomial sampling) on random-init 7B gptq.int4 weights, KV cache S = 2048.  Each decode step of the warm-up and timed
+loops reads its input token from a fixed seeded sequence instead of the previous step's sample (the sampling still runs
+on every step), so no step's input depends on how the build under test rounds.  The K timed steps are spread EVENLY over
 positions 16..2047 whatever K is (a stride, not consecutive positions), so `value` is a true ctx-2048 mean;
 `config.points` adds tokens/s at fixed positions 128, 1024 and 2047.  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the last timed step returned on rank 0, as float32 arrays: DIR/logits.npy (the model's
+(1, 1, 32000) logits) and DIR/token.npy (the sampled token).  Weights, prompt, input tokens and sampling noise are drawn
+from fixed seeds, so the same arguments give the same inputs on every run, and two builds that round differently give
+logits that differ by their rounding only (the token can differ only where that rounding decides a near-tie).
 
   value     tokens/s, device-timed (CUDA events), inputs resident in HBM, no host sync
   e2e       same loop driven from HOST buffers: per step a pinned H2D copy of the token and position, and a D2H read
@@ -379,6 +386,15 @@ def aggregate_throughput(world, steps, t_max):
     return world * steps / t_max
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -387,7 +403,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-tp", action="store_true", help="N > 1: skip the tensor-parallel block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's logits and token as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -404,6 +425,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     warm = max(3, args.warmup)
     K = args.steps
+    torch.manual_seed(1234 + rank)   # sampling noise (and any other default-generator draw): same arguments, same run
 
     model = build_synthetic_model(MODEL, dev, seed=1234)   # every replica holds the same weights, decodes its own stream
     compacted = False
@@ -412,6 +434,7 @@ def main():
         compacted = True
     gen = torch.Generator(device=dev).manual_seed(7 + rank)
     prompt = torch.randint(0, 32000, (PROMPT_T,), device=dev, dtype=torch.int32, generator=gen)
+    feed = torch.randint(0, 32000, (warm + K, 1, 1), device=dev, dtype=torch.int32, generator=gen)   # decode inputs
     lo, span = PROMPT_T, S_CTX - PROMPT_T
     # the K timed positions are spread evenly over [16, 2047] whatever K is (slots in between stay zero rows: the
     # attention kernel reads them exactly like written ones); warm-up walks the first positions
@@ -430,7 +453,7 @@ def main():
 
         # ---- value: device-resident loop, no host sync inside
         for i in range(warm):
-            tok = sample_next(model(tok.view(1, 1), S_CTX, pos_all[i])).to(torch.int32)
+            tok = sample_next(model(feed[i], S_CTX, pos_all[i])).to(torch.int32)
         barrier()
         clocks = ClockSampler(local)
         clocks.start()
@@ -439,12 +462,15 @@ def main():
         tw0 = time.time()
         e0.record()
         for i in range(warm, warm + K):
-            tok = sample_next(model(tok.view(1, 1), S_CTX, pos_all[i])).to(torch.int32)
+            logits = model(feed[i], S_CTX, pos_all[i])
+            tok = sample_next(logits).to(torch.int32)
         e1.record()
         barrier()
         tw1 = time.time()
         t_dev = e0.elapsed_time(e1) * 1e-3
         clk = clocks.stop(tw0, tw1)
+        if args.dump_outputs and rank == 0:   # nothing has run since the last timed step
+            dump_outputs(args.dump_outputs, {"logits": logits.float().cpu().numpy(), "token": tok.float().cpu().numpy()})
 
         # ---- e2e: host buffers; per step H2D (token, position) from pinned memory, D2H sampled token
         h_tok = torch.empty(1, dtype=torch.int32).pin_memory()

@@ -164,6 +164,23 @@ def golden_dense_model():
     torch.save(dict(cfg=cfg, seed=3, prompt=prompt, gen=y), os.path.join(OUT, "tiny_dense_f32.pt"))
 
 
+def golden_reference_layout():
+    """The public classes and functions of the reference modules lit_llama.patch_reference() rewires, with the module
+    each is defined in: tests/test_modules_cpu.py rebuilds a package of placeholders laid out the same way."""
+    import importlib
+    import json
+
+    layout = {}
+    for name in ("lit_llama", "lit_llama.model", "lit_llama.utils", "lit_llama.quantization", "generate"):
+        mod = importlib.import_module(name)
+        layout[name] = {k: v.__module__ for k, v in sorted(vars(mod).items())
+                        if not k.startswith("_") and callable(v)
+                        and str(getattr(v, "__module__", "")).split(".")[0] in ("lit_llama", "generate")}
+    with open(os.path.join(OUT, "reference_layout.json"), "w") as f:
+        json.dump(layout, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.manual_seed(0)
@@ -172,6 +189,7 @@ def main():
     golden_model(torch.float32, "f32")
     golden_model(torch.bfloat16, "bf16")
     golden_dense_model()
+    golden_reference_layout()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 

@@ -7,13 +7,11 @@ import sys
 import pytest
 import torch
 
-from conftest import load_golden
+from conftest import GOLDEN, load_golden
 
 import lit_llama_b200 as P
 from lit_llama_b200.utils import quantization
 from oracle import llama_oracle as O
-
-REF = "/root/reference"
 
 
 def test_find_multiple_and_lookup():
@@ -104,11 +102,41 @@ def test_product_does_not_import_the_oracle():
                 assert "oracle" not in src, f"{f} references oracle/"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
-def test_patch_reference_plugs_into_unmodified_reference():
-    here = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    sys.path.insert(0, os.path.join(here, "oracle", "_shim"))
-    sys.path.insert(0, REF)
+def _write_reference_standin(root, layout):
+    """A package laid out like the reference (tests/golden/reference_layout.json, recorded from it by
+    oracle/make_golden.py): every public class and function is a placeholder class in the module that defines it and
+    is imported by name into the modules that import it."""
+    defs, imports = {}, {}
+    for mod, names in layout.items():
+        for name, home in names.items():
+            defs.setdefault(home, set()).add(name)
+            if home != mod:
+                imports.setdefault(mod, []).append((home, name))
+    mods = set(defs) | set(imports)
+    pkgs = {m.rsplit(".", 1)[0] for m in mods if "." in m}
+    for mod in mods:
+        path = root.joinpath(*mod.split("."))
+        path = path / "__init__.py" if mod in pkgs else path.with_suffix(".py")
+        path.parent.mkdir(parents=True, exist_ok=True)
+        src = [f"from {home} import {name}" for home, name in sorted(imports.get(mod, []))]
+        src += [f"class {name}:\n    pass" for name in sorted(defs.get(mod, ()))]
+        path.write_text("\n".join(src) + "\n")
+
+
+def _reference_modules():
+    return [m for m in sys.modules if m in ("generate", "lit_llama") or m.startswith("lit_llama.")]
+
+
+def test_patch_reference_plugs_into_unmodified_reference(tmp_path, monkeypatch):
+    """patch_reference() on a package with the reference's module layout: the B200 classes replace the reference's
+    names everywhere a caller reaches them, including the names generate.py imported before the patch."""
+    import json
+
+    with open(os.path.join(GOLDEN, "reference_layout.json")) as f:
+        _write_reference_standin(tmp_path, json.load(f))
+    monkeypatch.syspath_prepend(str(tmp_path))
+    for name in _reference_modules():
+        monkeypatch.delitem(sys.modules, name)
     import lit_llama
     import lit_llama.quantization  # noqa: F401
     import generate as ref_generate
@@ -118,7 +146,7 @@ def test_patch_reference_plugs_into_unmodified_reference():
         from lit_llama.utils import quantization as ref_q
         from lit_llama.model import LLaMA as RefLLaMA, LLaMAConfig as RefCfg
 
-        assert RefLLaMA is P.LLaMA and ref_generate.LLaMA is P.LLaMA
+        assert RefLLaMA is P.LLaMA and ref_generate.LLaMA is P.LLaMA and ref_generate.quantization is quantization
         with ref_q("gptq.int4"):
             m = RefLLaMA(RefCfg(block_size=16, vocab_size=64, n_layer=1, n_head=2, n_embd=64))
         assert isinstance(m, P.LLaMA) and isinstance(m.lm_head, P.ColBlockQuantizedLinear)
@@ -132,6 +160,8 @@ def test_patch_reference_plugs_into_unmodified_reference():
                 setattr(tgt, name, val)
         ref_generate.LLaMA = saved[("model", "LLaMA")]
         ref_generate.quantization = saved[("utils", "quantization")]
+        for name in _reference_modules():
+            del sys.modules[name]
 
 
 def test_linear8bitlt_contract_on_cpu():
