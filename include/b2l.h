@@ -333,25 +333,13 @@ typedef struct b2l_decode_args {
   void* logits;              /* bf16 [B, vocab]                                       */
   int flags;                 /* B2L_F_*                                               */
   void* timeline;            /* debug: device uint64[(5*n_layer+1)*64] of %globaltimer stamps per
-                                launch (NULL = off); tools/diag.py `timeline`.  With `plan`: uint64
-                                [(5*n_layer+1)*16] per-op stamps of the persistent kernel   */
+                                launch (NULL = off); tools/diag.py `timeline`               */
   void* batch_work;          /* B in 2..8: scratch of b2l_q4_gemv_batch_workspace_bytes(max K) bytes; the
                                 linears then run on the mma.sync batch kernel (weights need qw_mma).
                                 NULL: tcgen05 kernel (weights need qw_tiled)              */
-  void* plan;                /* B == 1, head_size 128: device buffer of b2l_decode_plan_bytes() bytes prepared by
-                                b2l_decode_plan_build -> the whole step runs as ONE persistent kernel
-                                (csrc/decode_mega.cu; weights need the b2l_q4_tile_i8 layout in qw_mma).
-                                NULL: one kernel per op                                   */
 } b2l_decode_args;
 
 int b2l_decode_step(const b2l_decode_args* args, b2l_stream_t stream);
-/* The persistent decode kernel's static op list + arrival counters.  b2l_decode_plan_build fills args->plan from
- * the pointers in args (call it once, outside graph capture; rebuild when any pointer in args changes);
- * b2l_decode_plan_status synchronises the stream and returns B2L_E_STATE if a bounded wait inside the kernel
- * ever timed out (the kernel never hangs: it sets a sticky error word and falls through). */
-size_t b2l_decode_plan_bytes(const b2l_decode_args* args);
-int b2l_decode_plan_build(const b2l_decode_args* args, b2l_stream_t stream);
-int b2l_decode_plan_status(const void* plan, b2l_stream_t stream);
 /* Number of kernels one b2l_decode_step enqueues (for bench.py's gpu_launches). */
 int b2l_decode_step_launches(const b2l_decode_args* args);
 

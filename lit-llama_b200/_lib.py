@@ -54,7 +54,6 @@ class DecodeArgs(C.Structure):
         ("input_pos", c_void_p), ("ring_start", c_void_p), ("block_size", c_int),
         ("x", c_void_p), ("qkv", c_void_p), ("att", c_void_p), ("hid", c_void_p), ("attn_work", c_void_p),
         ("logits", c_void_p), ("flags", c_int), ("timeline", c_void_p), ("batch_work", c_void_p),
-        ("plan", c_void_p),
     ]
 
 
@@ -103,9 +102,6 @@ _SIGS = {
     "b2l_kv_unroll": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "b2l_decode_step": (c_int, [C.POINTER(DecodeArgs), c_void_p]),
     "b2l_decode_step_launches": (c_int, [C.POINTER(DecodeArgs)]),
-    "b2l_decode_plan_bytes": (c_size_t, [C.POINTER(DecodeArgs)]),
-    "b2l_decode_plan_build": (c_int, [C.POINTER(DecodeArgs), c_void_p]),
-    "b2l_decode_plan_status": (c_int, [c_void_p, c_void_p]),
 }
 
 EXPORTS = tuple(_SIGS)

@@ -10,7 +10,6 @@
 namespace b2l {
 
 extern void* g_attn_timeline;
-int decode_step_persistent(const b2l_decode_args* d, b2l_stream_t stream);   // decode_mega.cu
 
 static thread_local char g_err[512] = "";
 
@@ -154,7 +153,6 @@ static int q4_call(const b2l_q4_weight& w, const void* x, int ldx, void* y, int 
 
 extern "C" int b2l_decode_step_launches(const b2l_decode_args* d) {
   if (!d) return 0;
-  if (d->plan != nullptr) return 1;   // the persistent kernel
   const int attn = (d->n_embd / d->n_head == 128) ? 1 : 3;  // fused single-token attention for head_size 128
   const int lin = (d->B > 1 && d->B <= 8 && d->batch_work) ? 2 : 1;  // the batch kernel is two launches per linear
   return 2 + d->n_layer * (4 * lin + attn) + lin;  // ring advance + embedding, per Block 4 linears + attention, ln_f+lm_head
@@ -168,7 +166,6 @@ extern "C" int b2l_decode_step(const b2l_decode_args* d, b2l_stream_t stream) {
   B2L_CHECK_ARG(d->wte && d->ln_f && d->rope && d->idx && d->input_pos && d->ring_start && d->x && d->qkv && d->att &&
                     d->hid && d->attn_work && d->logits,
                 "b2l_decode_step: null pointer");
-  if (d->plan != nullptr) return decode_step_persistent(d, stream);   // one persistent kernel per token (decode_mega.cu)
   const int C = d->n_embd, hs = C / d->n_head, B = d->B;
   const int fl = d->flags;
   int rc;

@@ -361,8 +361,8 @@ extern "C" int b2l_debug_consumer_rate(void* out, int warps, int iters, int mode
 
 // ---- what does a grid-wide dependency cost without a kernel boundary?  Every CTA (all co-resident) arrives on a
 // global counter with red.release and polls it with ld.acquire until all have arrived; out[r] = max over CTAs of
-// the nanoseconds between its arrival and its release, out[rounds + r] = min.  The persistent-kernel plan of
-// DESIGN.md section 7 replaces five kernel boundaries per Block with five of these.
+// the nanoseconds between its arrival and its release, out[rounds + r] = min.  A kernel that fuses several ops
+// pays one of these for every kernel boundary it removes (DESIGN.md section 3 compares the two costs).
 __global__ void __launch_bounds__(128) grid_flag_kernel(unsigned long long* out, unsigned int* counter, int rounds) {
   if (threadIdx.x != 0) return;
   for (int r = 0; r < rounds; ++r) {

@@ -14,7 +14,6 @@ Two execution paths behind `LLaMA.forward`:
 """
 import ctypes as C
 import math
-import os
 from dataclasses import dataclass
 from typing import List, Optional, Tuple, Union
 
@@ -293,23 +292,11 @@ class _DecodeState:
             att=self.att.data_ptr(), hid=self.hid.data_ptr(), attn_work=self.work.data_ptr(),
             logits=self.logits.data_ptr(), flags=model.decode_flags,
             batch_work=None if self.batch_ws is None else self.batch_ws.data_ptr())
-        # batch 1, head_size 128: the whole step as ONE persistent kernel (csrc/decode_mega.cu)
-        self.plan = None
-        kmax = max(C_, n_hidden)
-        if model.persistent and B == 1 and hs == 128 and kmax <= 12288:
-            self.plan = torch.zeros(lib.b2l_decode_plan_bytes(C.byref(self.args)), dtype=torch.uint8, device=device)
-            self.args.plan = self.plan.data_ptr()
-            L.check(lib.b2l_decode_plan_build(C.byref(self.args), L.stream_ptr()), "b2l_decode_plan_build")
         self.graph: Optional[torch.cuda.CUDAGraph] = None
         self.calls = 0
 
     def enqueue(self) -> None:
         L.check(L.lib().b2l_decode_step(C.byref(self.args), L.stream_ptr()), "b2l_decode_step")
-
-    def check(self) -> None:
-        """Synchronises and raises if a bounded wait inside the persistent kernel ever timed out."""
-        if self.plan is not None:
-            L.check(L.lib().b2l_decode_plan_status(self.plan.data_ptr(), L.stream_ptr()), "b2l_decode_plan_status")
 
 
 class LLaMA(nn.Module):
@@ -321,10 +308,6 @@ class LLaMA(nn.Module):
     decode_flags: int = 1
     #: return a fresh logits tensor per call like the reference (False: a view of the static buffer)
     copy_logits: bool = True
-    #: batch-1 decode (head_size 128) as ONE persistent kernel per token (csrc/decode_mega.cu) instead of one kernel
-    #: per op.  Opt-in (B2L_PERSISTENT=1): measured on B200 it is correct but slower than the per-op path under
-    #: programmatic dependent launch (DESIGN.md section 4: 1330 vs 964 us per 7B token).
-    persistent: bool = os.environ.get("B2L_PERSISTENT", "0") == "1"
 
     def __init__(self, config: LLaMAConfig) -> None:
         super().__init__()

@@ -330,7 +330,7 @@ def test_fused_attention_equals_unfused(dev, S, cases):
 def test_fused_attention_vs_oracle_hs128(dev, B):
     """The kernel on the benched path (fused rope + KV append + split-S attention + merge, head_size 128) directly
     against the oracle's restatement of model.py:197-230 (O.rope_apply + index_copy / roll + O.sdpa): positions 0,
-    127, 128 (split boundary of the persistent kernel), 255, 256 (split boundary of this kernel), 1023, 2047 (full
+    127, 128 (sub-tile boundary of this kernel), 255, 256 (split boundary of this kernel), 1023, 2047 (full
     cache, 8 splits), and two roll states (model.py:214-218: position >= S with different ring offsets)."""
     from lit_llama_b200 import _lib as L
 

@@ -366,7 +366,7 @@ def test_int8_linear_vs_oracle(dev, N, K, M, outliers):
 def test_tp_allreduce_single_rank_is_identity(dev, n):
     """b2l_tp_allreduce with world = 1 (no peers): the multi-CTA indexing, the in-place path and the epoch words that
     advance in device memory -- the sum of one row is that row.  The peer exchange itself needs 2 GPUs
-    (tests/test_gpu_persistent.py::test_tensor_parallel_matches_single_gpu)."""
+    (tests/test_gpu_decode.py::test_tensor_parallel_matches_single_gpu)."""
     import ctypes as C
 
     from lit_llama_b200 import _lib as L

@@ -14,7 +14,7 @@ import time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-SECTIONS = ["generic", "tile", "tc_small", "tc_shapes", "tc_modes", "gemv", "mma_rate", "mma_issuers", "grid_flag", "hmma_rate", "imma_rate", "consumer_rate", "bench_gemm", "trace", "bench_layers", "bench_gemv", "bench_step", "bench_ctx", "bench_13b_b8", "bench_sizes", "batch_debug", "bench_step_int8", "timeline", "mega_timeline"]
+SECTIONS = ["generic", "tile", "tc_small", "tc_shapes", "tc_modes", "gemv", "mma_rate", "mma_issuers", "grid_flag", "hmma_rate", "imma_rate", "consumer_rate", "bench_gemm", "trace", "bench_layers", "bench_gemv", "bench_step", "bench_ctx", "bench_13b_b8", "bench_sizes", "batch_debug", "bench_step_int8", "timeline"]
 
 
 _DLIB = None
@@ -876,54 +876,6 @@ def sec_timeline():
             tot = int(t[n - 1, 4]) - int(t[0, 0])
             print(f"  whole step (first start -> lm_head end): {tot / 1e3:.1f} us; layer 4 start -> layer 5 start: "
                   f"{(int(t[25, 0]) - int(t[20, 0])) / 1e3:.2f} us")
-
-
-def sec_mega_timeline():
-    """Per-op %globaltimer stamps of the persistent decode kernel (7B, one eager step): where does an op's time go?"""
-    import torch
-    from bench import build_synthetic_model
-
-    dev = torch.device("cuda")
-    model = build_synthetic_model("7B", dev)
-    S = 2048
-    model.graph_after = 0
-    model.copy_logits = False
-    pos0 = int(os.environ.get("B2L_TL_POS", "64"))
-    with torch.no_grad():
-        model(torch.randint(0, 32000, (1, 16), device=dev, dtype=torch.int32), S, torch.arange(16, device=dev))
-        tok = torch.randint(0, 32000, (1, 1), device=dev, dtype=torch.int32)
-        for i in range(3):
-            model(tok, S, torch.tensor([pos0 + i], device=dev))
-        st = model._decode
-        assert st.plan is not None
-        n = 5 * model.config.n_layer + 1
-        tl = torch.zeros((n, 16), dtype=torch.int64, device=dev)
-        tl[:, 5] = 2**62
-        st.args.timeline = tl.data_ptr()
-        model(tok, S, torch.tensor([pos0 + 3], device=dev))
-        torch.cuda.synchronize()
-        st.args.timeline = None
-        st.check()
-    t = tl.cpu()
-    names = ["c_attn", "attn", "c_proj", "fc12", "mlp_proj"]
-    base = int(t[20, 5])
-    print(f"pos={pos0 + 3}; ns relative to layer 4 c_attn's first flag-seen: flag seen (min over CTAs) | CTA0 flag seen | CTA0 digits ready | "
-          "CTA0 loop done | loop done (max) | arrive (max)")
-    for li in range(20, 31):
-        v = [int(t[li, k]) for k in (5, 0, 1, 2, 3, 4)]
-        r = [x - base if x not in (0, 2**62) else None for x in v]
-        print(f"  L{li // 5} {names[li % 5]:9s} {r}   CTA0: consumer waited {int(t[li, 6]) / 1.965:.0f} ns for full stages, producer waited {int(t[li, 7]) / 1.965:.0f} ns for empty slots; "
-              f"units {int(t[li, 12])}, loop {int(t[li, 9]) / 1.965:.0f} ns of which scratch-free barrier {int(t[li, 8]) / 1.965:.0f} ns; epilogue warp {int(t[li, 11]) / 1.965:.0f} ns "
-              f"of which waiting for partials {int(t[li, 10]) / 1.965:.0f} ns")
-    print(f"  layer 4 -> layer 5 (flag seen min): {(int(t[25, 5]) - int(t[20, 5])) / 1e3:.2f} us;  whole step: "
-          f"{(int(t[n - 1, 4]) - int(t[0, 0])) / 1e3:.1f} us")
-    per = {}
-    for li in range(5, n - 1):
-        a, b = int(t[li, 5]), int(t[li + 1, 5])
-        per.setdefault(names[li % 5], []).append((b - a) / 1e3)
-    for k, v in per.items():
-        v = sorted(v)
-        print(f"  {k:9s}: flag-seen to next flag-seen us: median {v[len(v) // 2]:.2f} min {v[0]:.2f} max {v[-1]:.2f}")
 
 
 def sec_precision():
